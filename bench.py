@@ -7,6 +7,7 @@ one pass of the hot path over one such batch.  Weak scaling: every rank gets its
 
     python bench.py --gpus 1 --steps 200 --warmup 20           # this repo's CUDA path
     python bench.py --impl reference --steps 3 --warmup 1      # the CPU restatement of the reference path
+    python bench.py --steps 20 --dump-outputs DIR              # also write the last timed step's output as DIR/*.npy
     torchrun --nproc-per-node N bench.py --gpus N ...          # one rank per GPU
 
 Timing: the K steps (one mho_cheb_forward launch each, round-robin on --streams CUDA streams) are captured ONCE in a
@@ -243,6 +244,9 @@ def run_reference_arm(args):
         one_pass(cores)
     dt = time.perf_counter() - t0
     val = args.graphs * args.steps / dt
+    if args.dump_outputs:
+        Y = c_oracle.stack_forward(w["graph_off"], w["rowptr"], w["colidx"], None, ws, [2], 0.2, X64, cores)
+        dump_outputs(args.dump_outputs, {"Y": Y})
     out = {
         "impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
         "warmup": args.warmup, "ms_per_step": 1e3 * dt / args.steps, "higher_is_better": True, "scaling": "weak",
@@ -321,6 +325,23 @@ def bytes_of(w, survey=False):
     return 4 * n * F + 4 * n * F + 4 * (n + B) + (8 if survey else 4) * nnz
 
 
+DUMP_BYTES = 64 * 1024 * 1024
+
+
+def dump_outputs(out_dir, arrays, rank=0, world=1):
+    """Writes each array as out_dir/<name>.npy (<name>_rank<r>.npy under several ranks), so that two builds can be
+    compared output for output on the same seeded inputs.  Device tensors are written as float32, numpy arrays keep
+    float64.  All of them together stay within DUMP_BYTES: a larger array is cut to a fixed, seeded sample of its rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    budget = DUMP_BYTES // max(len(arrays), 1) - 4096   # (room for the .npy header)
+    for name, a in arrays.items():
+        a = np.asarray(a.detach().float().cpu().numpy() if hasattr(a, "detach") else a)
+        if a.nbytes > budget:
+            row_bytes = a.nbytes // a.shape[0]
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], size=budget // row_bytes, replace=False))]
+        np.save(os.path.join(out_dir, name + ("_rank%d" % rank if world > 1 else "") + ".npy"), a)
+
+
 def run_gpu_arm(args):
     import torch
     import torch.distributed as dist
@@ -335,6 +356,7 @@ def run_gpu_arm(args):
                          "(use --impl reference for the CPU restatement)")
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
+    torch.manual_seed(3 + rank)   # the rotating input sets: the same inputs on every run with the same arguments
     numa_node = bind_to_gpu_numa_node(torch, local)   # page-locked staging buffers land next to this rank's GPU
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
@@ -410,6 +432,8 @@ def run_gpu_arm(args):
         net.forward(batches[j], Xs[j], out=Ys[j])
         torch.cuda.synchronize()
         assert torch.equal(Ys[j], y), "overlapped step differs from a single launch"
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"Y": Ys[(args.steps - 1) % R]}, rank, world)
 
     # ---------------- e2e: host buffers in, host buffers out, through the C-ABI host call
     from multihop_offload_b200._lib import PinnedArray, pinned_like
@@ -637,7 +661,11 @@ def main():
     ap.add_argument("--no-pack", action="store_true", help="keep the random graph order instead of tile-packing order")
     ap.add_argument("--no-series", action="store_true", help="headline + e2e only")
     ap.add_argument("--sweep", default="compact", choices=["off", "compact", "full"], help="cfg-5 sweep: n x K (x B with 'full')")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (the layer output Y of the headline batch) as DIR/Y.npy, at most 64 MB")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference_arm(args)
     return run_gpu_arm(args)

@@ -1,6 +1,9 @@
 """Test doubles (tests/ only): an oracle-backed stand-in for ChebNet / KerasAdamReplay so that the HOST
 logic of the agent and drivers can be exercised on the CPU box against the reference's real simulator.
 The product never imports this; on a GPU the real libmho path is tested in test_agent_gpu.py."""
+import sys
+import types
+
 import numpy as np
 import scipy.sparse as sp
 import torch
@@ -116,3 +119,65 @@ def install(monkeypatch):
     monkeypatch.setattr(mod, "KerasAdamReplay", OracleAdam)
     monkeypatch.setattr(mod, "GraphBatch", FakeGraphBatch)
     return mod
+
+
+def install_apsp(monkeypatch):
+    """A ``util`` module whose all_pairs_shortest_paths (the reference's src/util.py:101-110, which the agent imports on the
+    CPU) is the oracle's Dijkstra, pinned bit for bit against the reference's own outputs in test_apsp.py."""
+    import apsp_oracle
+
+    def all_pairs_shortest_paths(graph, weight=None):
+        edges = list(graph.edges)
+        w = None if weight is None else [graph[a][b][weight] for a, b in edges]
+        return apsp_oracle.apsp_lengths(graph.number_of_nodes(), edges, w)
+
+    mod = types.ModuleType("util")
+    mod.all_pairs_shortest_paths = all_pairs_shortest_paths
+    monkeypatch.setitem(sys.modules, "util", mod)
+
+
+class RecordedStep:
+    """One forward_backward() step recorded against the reference's simulator (tests/golden/agent_case_n20.npz, written by
+    oracle/make_golden_agent.py): `obj` and `env` carry the fields the agent reads; env.offloading() checks that the agent
+    hands over the shortest-path matrices of the recording and sets the routes the simulator chose from them, env.run()
+    returns the recorded delays."""
+
+    def __init__(self, z):
+        import networkx as nx
+        self.z = z
+        n_ext = z["X"].shape[0]
+        A = sp.csr_matrix((z["gi_vals"], z["gi_colidx"], z["gi_rowptr"]), shape=(n_ext, n_ext))
+        self.adj, self.X = A, z["X"]
+        obj = types.SimpleNamespace(gi_ext=nx.from_scipy_sparse_array(A), num_edges_ext=n_ext,
+                                    edge_self_loop=z["X"][:, 0], edge_rate_ext=z["X"][:, 1], jobs_arrivals=z["X"][:, 2],
+                                    edge_as_server=z["X"][:, 3], maps_ol_el=z["maps_ol_el"], maps_on_el=z["maps_on_el"],
+                                    link_list_ext=[tuple(int(v) for v in e) for e in z["link_list_ext"]])
+        env = types.SimpleNamespace()
+        env.num_nodes, env.T, env.num_links = int(z["num_nodes"]), int(z["T"]), int(z["num_links"])
+        env.link_rates, env.cf_degs, env.proc_bws, env.link_matrix = z["link_rates"], z["cf_degs"], z["proc_bws"], z["link_matrix"]
+        L = env.num_links
+        env.adj_i = sp.csr_matrix((z["adj_i_vals"], z["adj_i_colidx"], z["adj_i_rowptr"]), shape=(L, L))
+        g = nx.Graph()
+        g.add_nodes_from(range(env.num_nodes))
+        g.add_edges_from([tuple(int(v) for v in e) for e in z["edges"]])
+        env.graph_c = g
+        env.num_jobs = len(z["job_source"])
+        env.jobs = [types.SimpleNamespace(source_node=int(s), arrival_rate=float(r), ul_data=float(u), dl_data=float(d))
+                    for s, r, u, d in zip(z["job_source"], z["job_rate"], z["job_ul"], z["job_dl"])]
+        env.flows = []
+        env.offloading, env.run = self.offloading, self.run
+        self.obj, self.env = obj, env
+
+    def offloading(self, sp_gnn, sp_hop, explore=0.0):
+        z = self.z
+        np.testing.assert_allclose(sp_gnn, z["sp_gnn"], rtol=1e-9, atol=0)
+        np.testing.assert_array_equal(sp_hop, z["sp_hop"])
+        assert explore == float(z["explore"])
+        off = z["flow_route_off"]
+        self.env.flows = [types.SimpleNamespace(dst=int(d), route=[int(v) for v in z["flow_route"][a:b]])
+                          for d, a, b in zip(z["flow_dst"], off[:-1], off[1:])]
+        return None, None
+
+    def run(self):
+        z = self.z
+        return z["delay_links"].copy(), z["delay_nodes"].copy(), z["delay_unit"].copy()

@@ -1,10 +1,11 @@
 """CPU: host logic of the drop-in agent and drivers against the reference's REAL simulator.
 
-Needs the reference checkout (skipped on the GPU box).  The GNN is an oracle-backed test double
-(tests/fakes.py); what is under test is everything around it: flags, feature assembly, queue head,
-bug-compatible delay matrix, environment coupling, critic, route gradient, VJP seeding, replay,
-checkpoints and the CSV schema.  The statistical pin replays the AdHoc_test protocol and compares
-mean tau of the GNN policy with the reference's shipped result CSV (SURVEY App. E/F)."""
+The GNN is an oracle-backed test double (tests/fakes.py); what is under test is everything around it: flags, feature
+assembly, queue head, bug-compatible delay matrix, environment coupling, critic, route gradient, VJP seeding, replay,
+checkpoints and the CSV schema.  One agent step is replayed from a recording made against the reference's simulator
+(tests/golden/agent_case_n20.npz); the tests that drive the simulator itself (the drivers, and the statistical pin that
+replays the AdHoc_test protocol and compares mean tau of the GNN policy with the reference's shipped result CSV, SURVEY
+App. E/F) need the reference checkout and skip without it."""
 import os
 import sys
 
@@ -16,7 +17,7 @@ import chebnet_oracle as O
 import fakes
 import ref_env
 
-pytestmark = pytest.mark.skipif(not ref_env.available(), reason="reference checkout not present")
+needs_reference = pytest.mark.skipif(not ref_env.available(), reason="drives the reference's simulator: reference checkout not present")
 REF = ref_env.REF_ROOT
 
 
@@ -32,29 +33,35 @@ def agent_mod(monkeypatch):
     F.fix_diag = False
     F.learning_rate = 1e-4
     F.training_set = "BAT800"
-    ref_env.import_env()
     return mod
 
 
-def _agent(mod, memory=1000):
+@pytest.fixture()
+def shipped(golden_dir):
+    """The reference's model_ChebConv_BAT800_a5_c5_ACO_agent (a byte copy, pinned in test_oracle.py)."""
+    return os.path.join(golden_dir, "ckpt_BAT800")
+
+
+def _agent(mod, ckpt, memory=1000):
     agent = mod.ACOAgent(mod.FLAGS, memory)
-    agent.load(os.path.join(REF, "model", "model_ChebConv_BAT800_a5_c5_ACO_agent"))
+    agent.load(ckpt)
     return agent
 
 
-def test_load_restores_shipped_weights_exactly(agent_mod):
-    agent = _agent(agent_mod)
-    ws = O.load_reference_weights(os.path.join(REF, "model", "model_ChebConv_BAT800_a5_c5_ACO_agent"))
+def test_load_restores_shipped_weights_exactly(agent_mod, shipped):
+    agent = _agent(agent_mod, shipped)
+    ws = O.load_reference_weights(shipped)
     for (W, b), (W2, b2) in zip(agent.net.get_weights(), ws):
         np.testing.assert_array_equal(W, W2); np.testing.assert_array_equal(b, b2)
     assert len(agent.model.trainable_weights) == 10
 
 
-def test_statistical_pin_forward_env(agent_mod):
+@needs_reference
+def test_statistical_pin_forward_env(agent_mod, shipped):
     """tau of the GNN policy, bug-compatible diagonal, vs the shipped CSV on the same network files."""
     from multihop_offload_b200.drivers_common import load_case, run_method, sample_jobs
     AdhocCloud, apsp = ref_env.import_env()
-    agent = _agent(agent_mod)
+    agent = _agent(agent_mod, shipped)
     datadir = os.path.join(REF, "data", "aco_data_ba_100")
     names = sorted(os.listdir(datadir))
     pick = names[::len(names) // 30][:30]
@@ -86,14 +93,15 @@ def test_statistical_pin_forward_env(agent_mod):
 
 
 @pytest.mark.slow
-def test_statistical_pin_150_files(agent_mod):
+@needs_reference
+def test_statistical_pin_150_files(agent_mod, shipped):
     """The same replay over 150 network files x 10 instances (SURVEY App. E's protocol; ~3 min on 8 cores): per-size tau
     table written to tests/golden/statistical_pin_150.json (committed), checked against the shipped CSV.
     Run with:  python -m pytest tests/test_agent_host.py -m slow -k 150 -s"""
     import json
     from multihop_offload_b200.drivers_common import load_case, run_method, sample_jobs
     AdhocCloud, apsp = ref_env.import_env()
-    agent = _agent(agent_mod)
+    agent = _agent(agent_mod, shipped)
     datadir = os.path.join(REF, "data", "aco_data_ba_100")
     names = sorted(os.listdir(datadir))
     pick = names[3::len(names) // 150][:150]
@@ -136,15 +144,12 @@ def test_statistical_pin_150_files(agent_mod):
         assert abs(g.tau_gnn.mean() - g.pub_gnn.mean()) < 2.5, (k, g.tau_gnn.mean(), g.pub_gnn.mean())
 
 
-def test_forward_backward_seeds_the_vjp_like_the_oracle(agent_mod):
-    from multihop_offload_b200.drivers_common import load_case, sample_jobs
-    AdhocCloud, apsp = ref_env.import_env()
-    agent = _agent(agent_mod)
-    fn = os.path.join(REF, "data", "aco_data_ba_10", "aco_case_seed500_m2_n20_s4.mat")
-    env, nodes_info, seed, n, m = load_case(AdhocCloud, fn, 1000)
-    np.random.seed(3)
-    sample_jobs(env, nodes_info, 0.15)
-    obj = env.graph_expand()
+def test_forward_backward_seeds_the_vjp_like_the_oracle(agent_mod, shipped, golden_dir, monkeypatch):
+    """One step on aco_case_seed500_m2_n20_s4.mat (jobs of np.random.seed(3)), replayed from the recording."""
+    fakes.install_apsp(monkeypatch)
+    agent = _agent(agent_mod, shipped)
+    step = fakes.RecordedStep(np.load(os.path.join(golden_dir, "agent_case_n20.npz")))
+    obj, env = step.obj, step.env
     captured = {}
     orig = agent.vjp_from_grad_dist
 
@@ -160,7 +165,7 @@ def test_forward_backward_seeds_the_vjp_like_the_oracle(agent_mod):
     gd = captured["gd"]
     assert gd.shape == (env.num_nodes, env.num_nodes) and np.isfinite(gd).all() and np.abs(gd).sum() > 0
     # independent restatement: oracle head VJP + oracle stack VJP on the same grad_dist
-    adj, X = ref_env.gnn_inputs(obj)
+    adj, X = step.adj, step.X
     ws = agent.net.get_weights()
     lam, cache = O.cheb_stack_forward(adj, X.astype(np.float32).astype(np.float64), ws, return_cache=True)
     ld, nd, hc = O.queue_head_forward(lam, obj.maps_ol_el, obj.maps_on_el, env.link_rates, env.cf_degs, env.proc_bws,
@@ -178,8 +183,8 @@ def test_forward_backward_seeds_the_vjp_like_the_oracle(agent_mod):
     assert np.abs(got - want).max() <= 1e-6 * max(np.abs(want).max(), 1e-30)
 
 
-def test_replay_applies_gradients_sequentially_and_checkpoints_roundtrip(agent_mod, tmp_path):
-    agent = _agent(agent_mod, memory=50)
+def test_replay_applies_gradients_sequentially_and_checkpoints_roundtrip(agent_mod, shipped, tmp_path):
+    agent = _agent(agent_mod, shipped, memory=50)
     rng = np.random.default_rng(0)
     import torch
     assert np.isnan(agent.replay(4))
@@ -198,6 +203,7 @@ def test_replay_applies_gradients_sequentially_and_checkpoints_roundtrip(agent_m
     np.testing.assert_array_equal(other.net.get_flat(), agent.net.get_flat())
 
 
+@needs_reference
 def test_adhoc_test_driver_csv_schema(agent_mod, tmp_path, monkeypatch):
     from multihop_offload_b200 import AdHoc_test
     monkeypatch.setattr(AdHoc_test, "ACOAgent", agent_mod.ACOAgent)
@@ -216,6 +222,7 @@ def test_adhoc_test_driver_csv_schema(agent_mod, tmp_path, monkeypatch):
     assert np.isfinite(df.tau).all()
 
 
+@needs_reference
 def test_adhoc_test_driver_batched_instances_same_rows(agent_mod, tmp_path, monkeypatch):
     """--batch_instances (SURVEY 8f #3): the GNN side of the 10 instances of a file is evaluated ahead of the per-instance
     loop without disturbing the random stream - every CSV row except the wall-clock column is identical."""
@@ -237,6 +244,7 @@ def test_adhoc_test_driver_batched_instances_same_rows(agent_mod, tmp_path, monk
     pd.testing.assert_frame_equal(dfs[0], dfs[1], check_exact=True)
 
 
+@needs_reference
 def test_adhoc_train_driver_replays_and_saves(agent_mod, tmp_path, monkeypatch):
     from multihop_offload_b200 import AdHoc_train, tf_bundle
     monkeypatch.setattr(AdHoc_train, "ACOAgent", agent_mod.ACOAgent)
