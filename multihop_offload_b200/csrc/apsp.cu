@@ -81,14 +81,5 @@ cudaError_t apsp_launch(int n_graphs, const int32_t* node_off, const int32_t* ro
     while ((size_t)(nodes + 1) * (nodes + 1) * 8 <= (size_t)max_smem_optin) ++nodes;
     p.smem_nodes = nodes;
     const size_t smem = (size_t)nodes * nodes * 8;
-    static int smem_set[64] = {0};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if ((int)smem > smem_set[dev & 63]) {
-        cudaError_t e = cudaFuncSetAttribute(apsp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        smem_set[dev & 63] = (int)smem;
-    }
-    apsp_kernel<<<n_graphs, APSP_THREADS, smem, st>>>(p);
-    return cudaGetLastError();
+    return mho_launch<apsp_kernel>(dim3((unsigned)n_graphs), dim3(APSP_THREADS), smem, st, false, p);
 }

@@ -338,32 +338,15 @@ static size_t bwd_smem_bytes(int rows_cap, int nnz_cap, int w_floats, bool has_v
 
 template <bool HAS_VALS, bool STAGED>
 static cudaError_t launch_bwd(const BwdParams& p, int grid, size_t smem, cudaStream_t st) {
-    auto kern = cheb_backward_kernel<HAS_VALS, STAGED>;
-    // the attribute is sticky per (function, device): only raise it when a launch needs more
-    static int smem_set[64] = {0};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if ((int)smem > smem_set[dev & 63]) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        smem_set[dev & 63] = (int)smem;
-    }
-    kern<<<grid, MHO_THREADS, smem, st>>>(p);
-    return cudaGetLastError();
+    return mho_launch<cheb_backward_kernel<HAS_VALS, STAGED>>(dim3((unsigned)grid), dim3(MHO_THREADS), smem, st, false, p);
 }
 
 extern "C" int mho_cheb_backward(mho_ctx_t* c, const mho_batch_t* b, const mho_layer_t* layers, int32_t n_layers,
                                  const float* X, const float* Y, const void* saved, const float* dY,
                                  float* grads_per_graph, float* grads_sum, float* dX, mho_stream_t stream) {
-    if (!c || !b || !layers) { mho_set_error("mho_cheb_backward: NULL argument"); return MHO_ERR_INVALID; }
-    if (n_layers < 1 || n_layers > MHO_MAX_LAYERS) { mho_set_error("mho_cheb_backward: n_layers=%d", n_layers); return MHO_ERR_INVALID; }
-    for (int l = 0; l < n_layers; ++l) {
-        const mho_layer_t& L = layers[l];
-        if (L.K < 1 || L.K > MHO_MAX_K || L.f_in < 1 || L.f_in > MHO_MAX_F || L.f_out < 1 || L.f_out > MHO_MAX_F || !L.W) {
-            mho_set_error("mho_cheb_backward: layer %d invalid", l);
-            return MHO_ERR_INVALID;
-        }
-    }
+    if (!c || !b) { mho_set_error("mho_cheb_backward: NULL argument"); return MHO_ERR_INVALID; }
+    int rc = validate_layers(layers, n_layers, "mho_cheb_backward");
+    if (rc) return rc;
     if (b->tile_off != nullptr) { mho_set_error("mho_cheb_backward: needs a one-graph-per-tile batch (tile_off == NULL)"); return MHO_ERR_INVALID; }
     if (!b->graph_off || !b->rowptr) { mho_set_error("mho_cheb_backward: invalid batch"); return MHO_ERR_INVALID; }
     const int64_t P = mho_param_count(layers, n_layers);
@@ -378,40 +361,25 @@ extern "C" int mho_cheb_backward(mho_ctx_t* c, const mho_batch_t* b, const mho_l
     if ((b->rowptr_t == nullptr) != (b->colidx_t == nullptr)) { mho_set_error("mho_cheb_backward: rowptr_t/colidx_t must both be set or both NULL"); return MHO_ERR_INVALID; }
     if (b->max_tile_rows < 1) { mho_set_error("mho_cheb_backward: batch.max_tile_rows must be the largest graph"); return MHO_ERR_INVALID; }
 
-    bool use_f16 = cheb_backward_f16_eligible(b, layers, n_layers, X, Y, dY, dX, c->max_smem_optin);
-    if (!use_f16 && cheb_mlp_backward_eligible(b, layers, n_layers, X, saved, dX, c->max_smem_optin)) {
-        // K = 1 stack (the shipped model): tensor-core VJP with cached W^T images
-        LayerDev ld[MHO_MAX_LAYERS];
-        mho_fill_layers(layers, n_layers, b->total_nodes, ld);
-        bool same = c->wmb_valid && (int)c->wbkey.size() == n_layers;
-        for (int l = 0; same && l < n_layers; ++l) {
-            const mho_wkey k{layers[l].W, layers[l].b, layers[l].K, layers[l].f_in, layers[l].f_out};
-            same = k == c->wbkey[l];
-        }
-        if (!same) {
-            const size_t bytes = (size_t)cheb_mlp_backward_weight_bytes(n_layers);
-            if (bytes > c->wmb_bytes) {
-                if (c->wmb) cudaFree(c->wmb);
-                c->wmb = nullptr; c->wmb_bytes = 0;
-                if (cudaMalloc((void**)&c->wmb, bytes) != cudaSuccess) { mho_set_error("cudaMalloc(%zu) for prepared weights failed", bytes); return MHO_ERR_CUDA; }
-                c->wmb_bytes = bytes;
-            }
-            cudaError_t e = cudaMemsetAsync(c->wmb, 0, bytes, st);
-            if (e == cudaSuccess) e = prepare_mlp_backward_weights_launch(ld, n_layers, c->wmb, st);
-            if (e != cudaSuccess) { mho_set_error("prepare_mlp_backward_weights launch failed: %s", cudaGetErrorString(e)); return MHO_ERR_CUDA; }
-            c->launches += 1;
-            c->wbkey.clear();
-            for (int l = 0; l < n_layers; ++l) c->wbkey.push_back(mho_wkey{layers[l].W, layers[l].b, layers[l].K, layers[l].f_in, layers[l].f_out});
-            c->wmb_valid = true;
-        }
-        cudaError_t e = cheb_mlp_backward_launch(b, ld, n_layers, X, Y, (const float*)saved, dY, grads_per_graph, (long long)P, c->wmb, c->num_sms, st);
-        if (e != cudaSuccess) { mho_set_error("cheb_mlp_backward launch failed: %s", cudaGetErrorString(e)); return MHO_ERR_CUDA; }
-        c->launches += 1;
-        use_f16 = true;   // (the per-graph rows are written: only the sum is left)
-    } else if (use_f16) {
+    // the tensor-core VJPs write the per-graph gradient rows; otherwise the CUDA-core kernel below does
+    bool rows_written = false;
+    if (cheb_backward_f16_eligible(b, layers, n_layers, X, Y, dY, dX, c->max_smem_optin)) {
         cudaError_t e = cheb_backward_f16_launch(b, layers, X, Y, dY, grads_per_graph, (long long)P, c->num_sms, st);
         if (e != cudaSuccess) { mho_set_error("cheb_backward_f16 launch failed: %s", cudaGetErrorString(e)); return MHO_ERR_CUDA; }
         c->launches += 1;
+        rows_written = true;
+    } else if (cheb_mlp_backward_eligible(b, layers, n_layers, X, saved, dX, c->max_smem_optin)) {
+        // K = 1 stack (the shipped model): tensor-core VJP with cached W^T images
+        LayerDev ld[MHO_MAX_LAYERS];
+        mho_fill_layers(layers, n_layers, b->total_nodes, ld);
+        auto& img = c->img[MHO_IMG_MLP_BWD];
+        rc = ensure_image(c, img, layers, n_layers, (size_t)cheb_mlp_backward_weight_bytes(n_layers), "prepare_mlp_backward_weights",
+                          [&](unsigned char* out) { return prepare_mlp_backward_weights_launch(ld, n_layers, out, st); });
+        if (rc) return rc;
+        cudaError_t e = cheb_mlp_backward_launch(b, ld, n_layers, X, Y, (const float*)saved, dY, grads_per_graph, (long long)P, img.ptr, c->num_sms, st);
+        if (e != cudaSuccess) { mho_set_error("cheb_mlp_backward launch failed: %s", cudaGetErrorString(e)); return MHO_ERR_CUDA; }
+        c->launches += 1;
+        rows_written = true;
     }
     BwdParams p;
     memset(&p, 0, sizeof(p));
@@ -449,11 +417,12 @@ extern "C" int mho_cheb_backward(mho_ctx_t* c, const mho_batch_t* b, const mho_l
     int grid = c->num_sms * per_sm;
     if (grid > b->n_graphs) grid = b->n_graphs;
     cudaError_t e = cudaSuccess;
-    if (use_f16) { /* done above */ }
-    else if (has_vals) e = staged ? launch_bwd<true, true>(p, grid, smem, st) : launch_bwd<true, false>(p, grid, smem, st);
-    else e = staged ? launch_bwd<false, true>(p, grid, smem, st) : launch_bwd<false, false>(p, grid, smem, st);
-    if (e != cudaSuccess) { mho_set_error("cheb_backward launch failed: %s", cudaGetErrorString(e)); return MHO_ERR_CUDA; }
-    if (!use_f16) c->launches += 1;
+    if (!rows_written) {
+        if (has_vals) e = staged ? launch_bwd<true, true>(p, grid, smem, st) : launch_bwd<true, false>(p, grid, smem, st);
+        else e = staged ? launch_bwd<false, true>(p, grid, smem, st) : launch_bwd<false, false>(p, grid, smem, st);
+        if (e != cudaSuccess) { mho_set_error("cheb_backward launch failed: %s", cudaGetErrorString(e)); return MHO_ERR_CUDA; }
+        c->launches += 1;
+    }
     if (grads_sum) {
         const int threads = 128;
         const bool vec4 = (P % 4 == 0) && ((reinterpret_cast<uintptr_t>(grads_per_graph) | reinterpret_cast<uintptr_t>(grads_sum)) & 15u) == 0;

@@ -494,9 +494,6 @@ __global__ void __launch_bounds__(BF_THREADS, 2) cheb_backward_f16_kernel(const 
 // -------------------------------------------------------------------------------------------
 bool cheb_backward_f16_eligible(const mho_batch_t* b, const mho_layer_t* layers, int n_layers, const void* X, const void* Y, const void* dY,
                                 const void* dX, int max_smem_optin) {
-    static int dbg = -1;
-    if (dbg < 0) { const char* e = getenv("MHO_DEBUG"); dbg = e ? atoi(e) : 0; }
-    if (dbg & 512) return false;   // MHO_DEBUG & 512: keep the CUDA-core VJP
     if (n_layers != 1 || dX != nullptr || b->vals != nullptr || b->adj_bits == nullptr || b->max_tile_rows > 128) return false;
     const mho_layer_t& L = layers[0];
     if (L.f_in != 32 || L.f_out != 32 || L.K < 2 || L.K > 10) return false;
@@ -520,17 +517,7 @@ cudaError_t cheb_backward_f16_launch(const mho_batch_t* b, const mho_layer_t* la
     p.act = layers[0].act;
     p.slope = layers[0].slope;
     const size_t smem = (size_t)BF_SMEM + 1024;
-    static int smem_set[64] = {0};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (!smem_set[dev & 63]) {
-        cudaError_t e = cudaFuncSetAttribute(cheb_backward_f16_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(cheb_backward_f16_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        smem_set[dev & 63] = 1;
-    }
-    int grid = std::min(2 * num_sms, std::max(1, p.n_graphs));
-    if (p.K > 6) cheb_backward_f16_kernel<true><<<grid, BF_THREADS, smem, st>>>(p);     // running-maximum scales
-    else cheb_backward_f16_kernel<false><<<grid, BF_THREADS, smem, st>>>(p);
-    return cudaGetLastError();
+    const dim3 grid((unsigned)std::min(2 * num_sms, std::max(1, p.n_graphs)));
+    if (p.K > 6) return mho_launch<cheb_backward_f16_kernel<true>>(grid, dim3(BF_THREADS), smem, st, false, p);   // running-maximum scales
+    return mho_launch<cheb_backward_f16_kernel<false>>(grid, dim3(BF_THREADS), smem, st, false, p);
 }

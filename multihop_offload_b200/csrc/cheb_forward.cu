@@ -19,9 +19,6 @@
 //     3xTF32 split in registers for fp32-grade accuracy) straight out of the same tiles via
 //     ldmatrix, interleaved with the sparse step for T_{k+1};
 //   * HBM traffic per tile is exactly X in, Y out, CSR once; T_k never leaves the SM.
-#include <cstdlib>
-#include <cstring>
-
 #include "mho_common.cuh"
 
 // the forward kernel runs 16 warps per CTA: two CTAs per SM then give 32 resident warps, which this
@@ -555,7 +552,7 @@ cheb_forward_kernel(const __grid_constant__ FwdParams p) {
             for (int k = 0; k < L.K; ++k) {
                 const uint32_t whi_k = w_l + (uint32_t)(k * fo_img) * 128u;
                 const uint32_t wlo_k = whi_k + (uint32_t)w_rows_l * 128u;
-                const bool more = (k + 1 < L.K) && !(p.debug & 1);
+                const bool more = k + 1 < L.K;
                 HeadState hs;
                 hs.pending = 0;
                 if (TC5) {
@@ -606,7 +603,7 @@ cheb_forward_kernel(const __grid_constant__ FwdParams p) {
                 }
                 // the dense contribution of T_k right behind the walk: warps that finish their segment early
                 // start on the tensor cores, so one barrier absorbs the imbalance of both
-                if (has_n && !(p.debug & 2)) {
+                if (has_n) {
 #pragma unroll
                     for (int m = 0; m < MT; ++m) {
                         const int mt = mslot + m * FWD_MSLOTS;
@@ -731,28 +728,7 @@ static size_t fwd_smem_bytes(int rows_cap, int nnz_cap, int w_rows, bool has_val
 
 template <int MT, bool HAS_VALS, bool STAGED, bool TC5 = false>
 static cudaError_t launch_one(const FwdParams& p, int grid, size_t smem, cudaStream_t st) {
-    auto kern = cheb_forward_kernel<MT, HAS_VALS, STAGED, TC5>;
-    // the attribute is sticky per (function, device): only raise it when a launch needs more
-    static int smem_set[64] = {0};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if ((int)smem > smem_set[dev & 63]) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        smem_set[dev & 63] = (int)smem;
-    }
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = dim3((unsigned)grid);
-    cfg.blockDim = dim3(FWD_THREADS);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, kern, p);
+    return mho_launch<cheb_forward_kernel<MT, HAS_VALS, STAGED, TC5>>(dim3((unsigned)grid), dim3(FWD_THREADS), smem, st, true, p);
 }
 
 template <int MT>
@@ -784,26 +760,23 @@ cudaError_t cheb_forward_launch(FwdParams& p, int max_tile_rows, int max_tile_nn
     p.w_rows_cap = p.w_resident ? w_sum : w_max;
     if (!p.w_resident) for (int l = 0; l < p.n_layers; ++l) p.w_row_off[l] = 0;
 
-    static int dbg = -1;
-    if (dbg < 0) { const char* e = getenv("MHO_DEBUG"); dbg = e ? atoi(e) : 0; }
-    p.debug = dbg;
     // preference order: tcgen05 dense path (one 128-row M tile, no prefetch buffer), then
     // staged+prefetch with >=2 CTAs/SM, staged+prefetch, staged, global CSR
     const int nnz_cap = (max_tile_nnz + 3) & ~3;
     bool staged = true, prefetch = true, tc5 = false;
     auto per_sm_of = [&](size_t s) { int v = (int)((size_t)(228 * 1024) / (s + 1024)); return v > reg_limit ? reg_limit : v; };
     size_t smem = 0;
-    if (mt_sel == 1 && !(dbg & 16)) {
+    if (mt_sel == 1) {
         p.rows_cap = 128;  // the UMMA M extent
         const size_t s5p = fwd_smem_bytes(128, nnz_cap, p.w_rows_cap, has_vals, true, true);
         const size_t s5 = fwd_smem_bytes(128, nnz_cap, p.w_rows_cap, has_vals, false, true);
-        if (s5p <= (size_t)max_smem_optin && per_sm_of(s5p) >= 2 && !(dbg & 8)) { tc5 = true; prefetch = true; smem = s5p; }
+        if (s5p <= (size_t)max_smem_optin && per_sm_of(s5p) >= 2) { tc5 = true; prefetch = true; smem = s5p; }
         else if (s5 <= (size_t)max_smem_optin) { tc5 = true; prefetch = false; smem = s5; }
     }
     if (!tc5) {
         smem = fwd_smem_bytes(p.rows_cap, nnz_cap, p.w_rows_cap, has_vals, true, false);
         const size_t smem_np = fwd_smem_bytes(p.rows_cap, nnz_cap, p.w_rows_cap, has_vals, false, false);
-        if (smem > (size_t)max_smem_optin || (per_sm_of(smem) < 2 && per_sm_of(smem_np) >= 2 && reg_limit >= 2) || (dbg & 8)) {
+        if (smem > (size_t)max_smem_optin || (per_sm_of(smem) < 2 && per_sm_of(smem_np) >= 2 && reg_limit >= 2)) {
             prefetch = false;
             smem = smem_np;
         }

@@ -582,9 +582,6 @@ __global__ void __launch_bounds__(DN_THREADS, 2) cheb_dense_kernel(const __grid_
 // -------------------------------------------------------------------------------------------
 bool cheb_dense_eligible(const mho_layer_t* layers, int n_layers, bool has_vals, bool has_bits, int max_tile_rows, int max_tile_nnz,
                          int max_smem_optin) {
-    static int dbg = -1;
-    if (dbg < 0) { const char* e = getenv("MHO_DEBUG"); dbg = e ? atoi(e) : 0; }
-    if (dbg & 32) return false;  // MHO_DEBUG & 32: keep the CSR-walk kernel
     if (max_tile_rows > 128) return false;
     int wb = 0;
     bool need_adj = false;
@@ -615,6 +612,10 @@ cudaError_t prepare_dense_weights_launch(const LayerDev* layers, int n_layers, c
     p.n_layers = n_layers;
     for (int l = 0; l < n_layers; ++l) { p.layers[l] = layers[l]; p.w_off[l] = w_off[l]; }
     p.out = out;
+    // the kernel writes the weight parts and bias rows, not the padding of each layer's block
+    const int bytes = w_off[n_layers - 1] + dn_layer_bytes(layers[n_layers - 1].K, layers[n_layers - 1].f_out);
+    const cudaError_t e = cudaMemsetAsync(out, 0, (size_t)bytes, st);
+    if (e != cudaSuccess) return e;
     dim3 grid(8, n_layers);
     prepare_dense_weights_kernel<<<grid, 256, 0, st>>>(p);
     return cudaGetLastError();
@@ -652,29 +653,8 @@ cudaError_t cheb_dense_launch(const FwdParams& fp, const unsigned char* wimg, co
     p.w_slot = wmax;
     p.w_bytes = p.w_resident ? w_bytes : 2 * wmax;
     const size_t smem = rest + (size_t)p.w_bytes;
-    static int smem_set[64] = {0};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if ((int)smem > smem_set[dev & 63]) {
-        cudaError_t e = cudaFuncSetAttribute(cheb_dense_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        smem_set[dev & 63] = (int)smem;
-    }
     int grid = num_sms * 2;
     if (grid > p.b.n_tiles) grid = p.b.n_tiles;
     if (grid < 1) grid = 1;
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = dim3((unsigned)grid);
-    cfg.blockDim = dim3(DN_THREADS);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    static int no_pdl = -1;
-    if (no_pdl < 0) { const char* e = getenv("MHO_NO_PDL"); no_pdl = e ? atoi(e) : 0; }
-    cfg.numAttrs = no_pdl ? 0 : 1;
-    return cudaLaunchKernelEx(&cfg, cheb_dense_kernel, p);
+    return mho_launch<cheb_dense_kernel>(dim3((unsigned)grid), dim3(DN_THREADS), smem, st, true, p);
 }

@@ -56,7 +56,6 @@ struct HfParams {
     const unsigned char* wimg;  // [32 K rows x 128 B: W'_k[o][f] as fp16 h | l][bias row 128 B][header 128 B]
     int act;
     float slope;
-    int stagger;      // clock cycles the second CTA of an SM waits before its first tile (de-phases the two CTAs)
     int use_bits;     // the batch carries adjacency bit rows
     int nnz_cap;      // CSR staging capacity in ints (multiple of 4), 0 with bit rows
     int stage_bytes;  // bytes of one operator staging set (multiple of 16)
@@ -129,9 +128,10 @@ __global__ void __launch_bounds__(256) hf_prepare_weights_kernel(const HfPrepPar
 //   epilogue of the previous tile and this tile's adjacency expansion run under the X W group;
 //   X W done -> scales, B_K-1 = P_K-1 / row scale, split, arrive;   next tile's input rows are split into the OTHER part
 //   tile inside the wait window of a Clenshaw step;   steps k = K-2 .. 0: wait, LDTM, recurrence (packed fp32), split, arrive.
-template <int K, bool TRACK>
+template <int K>
 __global__ void __launch_bounds__(HF_THREADS, (K <= 5 ? 2 : 1)) cheb_f16_kernel(const __grid_constant__ HfParams p) {
     extern __shared__ __align__(1024) unsigned char smem[];
+    constexpr bool TRACK = K > 5;   // Clenshaw step scales from the running maxima of |B_k| (K <= 5: the a-priori bounds suffice)
     constexpr int W_BYTES = hf_w_bytes(K);
     constexpr uint32_t TCOLS = (K <= 5) ? 256u : 512u;
     constexpr uint32_t ADJ_COL = TCOLS - 64u;
@@ -439,10 +439,6 @@ __global__ void __launch_bounds__(HF_THREADS, (K <= 5 ? 2 : 1)) cheb_f16_kernel(
             arrive_issue(buf, step, rows_t);
         };
 
-        if (p.stagger > 0 && (int)blockIdx.x >= (G + 1) / 2) {
-            const long long t0 = clock64();
-            while (clock64() - t0 < (long long)p.stagger) { }
-        }
         if (n_my > 0) {
             x_split(0, 2);
             arrive_issue(0, -1, 0);   // (the first tile's bit rows, built by all threads, are read behind the barrier at the top of the tile loop)
@@ -1132,54 +1128,12 @@ __global__ void __launch_bounds__(384, 2) cheb_f16ws_kernel(const __grid_constan
 
 template <int K, bool S_SPLIT>
 cudaError_t launch_ws(const HfParams& p, size_t smem, int grid, cudaStream_t st) {
-    static int smem_set[64] = {0};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if ((int)smem > smem_set[dev & 63]) {
-        cudaError_t e = cudaFuncSetAttribute(cheb_f16ws_kernel<K, S_SPLIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        smem_set[dev & 63] = (int)smem;
-    }
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = dim3((unsigned)grid);
-    cfg.blockDim = dim3(384);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    static int no_pdl = -1;
-    if (no_pdl < 0) { const char* e = getenv("MHO_NO_PDL"); no_pdl = e ? atoi(e) : 0; }
-    cfg.numAttrs = no_pdl ? 0 : 1;
-    return cudaLaunchKernelEx(&cfg, cheb_f16ws_kernel<K, S_SPLIT>, p);
+    return mho_launch<cheb_f16ws_kernel<K, S_SPLIT>>(dim3((unsigned)grid), dim3(384), smem, st, true, p);
 }
 
-template <int K, bool TRACK>
+template <int K>
 cudaError_t launch_k(const HfParams& p, size_t smem, int grid, cudaStream_t st) {
-    static int smem_set[64] = {0};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if ((int)smem > smem_set[dev & 63]) {
-        cudaError_t e = cudaFuncSetAttribute(cheb_f16_kernel<K, TRACK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        smem_set[dev & 63] = (int)smem;
-    }
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = dim3((unsigned)grid);
-    cfg.blockDim = dim3(HF_THREADS);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    static int no_pdl = -1;
-    if (no_pdl < 0) { const char* e = getenv("MHO_NO_PDL"); no_pdl = e ? atoi(e) : 0; }
-    cfg.numAttrs = no_pdl ? 0 : 1;
-    return cudaLaunchKernelEx(&cfg, cheb_f16_kernel<K, TRACK>, p);
+    return mho_launch<cheb_f16_kernel<K>>(dim3((unsigned)grid), dim3(HF_THREADS), smem, st, true, p);
 }
 
 }  // namespace
@@ -1196,9 +1150,6 @@ static size_t hf_smem_bytes(int K, bool has_bits, int max_tile_nnz, int* stage_b
 
 bool cheb_f16_eligible(const mho_layer_t* layers, int n_layers, bool has_vals, bool has_bits, bool has_saved, bool has_graph_starts,
                        int max_tile_rows, int max_tile_nnz, const void* X, const void* Y, const void* bits, int max_smem_optin) {
-    static int dbg = -1;
-    if (dbg < 0) { const char* e = getenv("MHO_DEBUG"); dbg = e ? atoi(e) : 0; }
-    if (dbg & (32 | 64)) return false;   // MHO_DEBUG & 64: keep the first-generation dense kernel; & 32: the CSR-walk kernel
     // one scale per tile is exact to 1e-5 only while tile mates stay within ~2^7 of each other in magnitude at every Clenshaw
     // step: without the graph starts (mho_batch_t.tile_graph0) the batch goes to the bf16 x 3 kernel, which needs no scales
     if (n_layers != 1 || has_vals || has_saved || !has_graph_starts || max_tile_rows > 128) return false;
@@ -1214,6 +1165,9 @@ int cheb_f16_weight_bytes(int K) { return hf_w_bytes(K); }
 
 cudaError_t prepare_f16_weights_launch(const LayerDev& L, unsigned char* out, cudaStream_t st) {
     HfPrepParams p{L.W, L.b, L.K, out};
+    // the kernel writes the weight rows, bias and header, not the padding up to hf_w_bytes
+    const cudaError_t e = cudaMemsetAsync(out, 0, (size_t)hf_w_bytes(L.K), st);
+    if (e != cudaSuccess) return e;
     hf_prepare_weights_kernel<<<1, 256, 0, st>>>(p);
     return cudaGetLastError();
 }
@@ -1228,22 +1182,15 @@ cudaError_t cheb_f16_launch(const FwdParams& fp, const unsigned char* wimg, int 
     p.act = fp.layers[0].act;
     p.slope = fp.layers[0].slope;
     p.use_bits = fp.b.adj_bits != nullptr ? 1 : 0;
-    static int stagger_env = -1;
-    if (stagger_env < 0) { const char* e = getenv("MHO_STAGGER"); stagger_env = e ? atoi(e) : 0; }
-    p.stagger = stagger_env;
     const int K = fp.layers[0].K;
     int stage = 0;
-    static int track_env = -1;
-    if (track_env < 0) { const char* e = getenv("MHO_TRACK"); track_env = e ? atoi(e) : 0; }   // 1: running-maximum scales for every K
     p.nnz_cap = p.use_bits ? 0 : ((max_tile_nnz + 3) & ~3);
     const size_t smem = hf_smem_bytes(K, p.use_bits != 0, max_tile_nnz, &stage);
     p.stage_bytes = stage;
     int grid = num_sms * (K <= 5 ? 2 : 1);   // (one CTA per SM per launch + more streams was measured: no gain)
     if (grid > p.b.n_tiles) grid = p.b.n_tiles;
     if (grid < 1) grid = 1;
-    static int ws_env = -1;
-    if (ws_env < 0) { const char* e = getenv("MHO_WS"); ws_env = e ? atoi(e) : 1; }   // MHO_WS=0: the eight-warp kernel for every shape
-    if (ws_env && K <= 5 && p.use_bits && p.b.tile_graph0 != nullptr && !track_env) {
+    if (K <= 5 && p.use_bits && p.b.tile_graph0 != nullptr) {
         switch (K) {
             // who splits the next tile's rows: the compute warps inside their wait windows (short tiles: the 96 service threads need
             // ~7 k cycles for a tile's rows), or the service warps (K >= 4: 5 % faster on the benchmark layer)
@@ -1254,15 +1201,15 @@ cudaError_t cheb_f16_launch(const FwdParams& fp, const unsigned char* wimg, int 
         }
     }
     switch (K) {
-        case 2: return track_env ? launch_k<2, true>(p, smem, grid, st) : launch_k<2, false>(p, smem, grid, st);
-        case 3: return track_env ? launch_k<3, true>(p, smem, grid, st) : launch_k<3, false>(p, smem, grid, st);
-        case 4: return track_env ? launch_k<4, true>(p, smem, grid, st) : launch_k<4, false>(p, smem, grid, st);
-        case 5: return track_env ? launch_k<5, true>(p, smem, grid, st) : launch_k<5, false>(p, smem, grid, st);
-        case 6: return launch_k<6, true>(p, smem, grid, st);
-        case 7: return launch_k<7, true>(p, smem, grid, st);
-        case 8: return launch_k<8, true>(p, smem, grid, st);
-        case 9: return launch_k<9, true>(p, smem, grid, st);
-        case 10: return launch_k<10, true>(p, smem, grid, st);
+        case 2: return launch_k<2>(p, smem, grid, st);
+        case 3: return launch_k<3>(p, smem, grid, st);
+        case 4: return launch_k<4>(p, smem, grid, st);
+        case 5: return launch_k<5>(p, smem, grid, st);
+        case 6: return launch_k<6>(p, smem, grid, st);
+        case 7: return launch_k<7>(p, smem, grid, st);
+        case 8: return launch_k<8>(p, smem, grid, st);
+        case 9: return launch_k<9>(p, smem, grid, st);
+        case 10: return launch_k<10>(p, smem, grid, st);
         default: return cudaErrorInvalidValue;
     }
 }

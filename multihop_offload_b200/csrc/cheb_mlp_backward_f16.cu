@@ -403,9 +403,6 @@ size_t mb_smem_bytes(int n_layers) {
 // -------------------------------------------------------------------------------------------
 bool cheb_mlp_backward_eligible(const mho_batch_t* b, const mho_layer_t* layers, int n_layers, const void* X, const void* saved, const void* dX,
                                 int max_smem_optin) {
-    static int dbg = -1;
-    if (dbg < 0) { const char* e = getenv("MHO_DEBUG"); dbg = e ? atoi(e) : 0; }
-    if (dbg & 2048) return false;   // MHO_DEBUG & 2048: keep the CUDA-core VJP for K = 1 stacks
     if (n_layers < 2 || n_layers > MB_MAX_LAYERS || dX != nullptr || saved == nullptr || b->max_tile_rows > 128) return false;
     for (int l = 0; l < n_layers; ++l) {
         if (layers[l].K != 1) return false;
@@ -425,6 +422,9 @@ cudaError_t prepare_mlp_backward_weights_launch(const LayerDev* layers, int n_la
     p.n_layers = n_layers;
     for (int l = 0; l < n_layers; ++l) p.layers[l] = layers[l];
     p.out = out;
+    // the kernel writes the W^T rows, not the padding of each layer's block
+    const cudaError_t e = cudaMemsetAsync(out, 0, (size_t)n_layers * MB_WT_BYTES, st);
+    if (e != cudaSuccess) return e;
     mlpT_prepare_weights_kernel<<<n_layers, 256, 0, st>>>(p);
     return cudaGetLastError();
 }
@@ -445,15 +445,6 @@ cudaError_t cheb_mlp_backward_launch(const mho_batch_t* b, const LayerDev* layer
         p.saved_off[l] = layers[l].saved_off; p.param_off[l] = layers[l].param_off;
     }
     const size_t smem = mb_smem_bytes(n_layers) + 1024;
-    static int smem_set[64] = {0};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if ((int)smem > smem_set[dev & 63]) {
-        cudaError_t e = cudaFuncSetAttribute(cheb_mlp_backward_f16_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        smem_set[dev & 63] = (int)smem;
-    }
-    int grid = std::min(2 * num_sms, std::max(1, p.n_graphs));
-    cheb_mlp_backward_f16_kernel<<<grid, MB_THREADS, smem, st>>>(p);
-    return cudaGetLastError();
+    const int grid = std::min(2 * num_sms, std::max(1, p.n_graphs));
+    return mho_launch<cheb_mlp_backward_f16_kernel>(dim3((unsigned)grid), dim3(MB_THREADS), smem, st, false, p);
 }

@@ -289,9 +289,6 @@ static size_t mlp_smem_bytes(int n_layers, int f_in0, bool stage) {
 }
 
 bool cheb_mlp_eligible(const mho_layer_t* layers, int n_layers, int max_tile_rows, const void* X, int max_smem_optin) {
-    static int dbg = -1;
-    if (dbg < 0) { const char* e = getenv("MHO_DEBUG"); dbg = e ? atoi(e) : 0; }
-    if (dbg & (32 | 64 | 256)) return false;   // MHO_DEBUG & 256: keep the first-generation dense kernel for K = 1 stacks
     if (max_tile_rows > 128 || n_layers < 1) return false;
     for (int l = 0; l < n_layers; ++l)
         if (layers[l].K != 1 || layers[l].f_in > 32 || layers[l].f_out > 32) return false;
@@ -329,29 +326,8 @@ cudaError_t cheb_mlp_launch(const FwdParams& fp, const unsigned char* wimg, int 
     for (int l = 0; l + 1 < fp.n_layers; ++l) stage = stage || (fp.saved != nullptr && fp.layers[l].f_out == 32);
     p.stage_bytes = stage ? HF_TILE_BYTES : 0;
     const size_t smem = mlp_smem_bytes(fp.n_layers, p.f_in0, stage);
-    static int smem_set[64] = {0};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if ((int)smem > smem_set[dev & 63]) {
-        cudaError_t e = cudaFuncSetAttribute(cheb_mlp_f16_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        smem_set[dev & 63] = (int)smem;
-    }
     int per_sm = (int)((size_t)(227 * 1024) / (smem + 1024));
     per_sm = std::max(1, std::min(per_sm, 4));
     int grid = std::min(num_sms * per_sm, std::max(1, p.b.n_tiles));
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = dim3((unsigned)grid);
-    cfg.blockDim = dim3(MLP_THREADS);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    static int no_pdl = -1;
-    if (no_pdl < 0) { const char* e = getenv("MHO_NO_PDL"); no_pdl = e ? atoi(e) : 0; }
-    cfg.numAttrs = no_pdl ? 0 : 1;
-    return cudaLaunchKernelEx(&cfg, cheb_mlp_f16_kernel, p);
+    return mho_launch<cheb_mlp_f16_kernel>(dim3((unsigned)grid), dim3(MLP_THREADS), smem, st, true, p);
 }

@@ -71,11 +71,7 @@ extern "C" int mho_destroy(mho_ctx_t* c) {
     if (!c) return MHO_OK;
     cudaSetDevice(c->device);
     for (auto& s : c->scratch) if (s.ptr) cudaFree(s.ptr);
-    if (c->wprep) cudaFree(c->wprep);
-    if (c->wdense) cudaFree(c->wdense);
-    if (c->wf16) cudaFree(c->wf16);
-    if (c->wmlp) cudaFree(c->wmlp);
-    if (c->wmb) cudaFree(c->wmb);
+    for (auto& im : c->img) if (im.ptr) cudaFree(im.ptr);
     if (c->sched) cudaFree(c->sched);
     if (c->h2d_stream) {
         cudaStreamDestroy(c->h2d_stream); cudaStreamDestroy(c->d2h_stream);
@@ -111,100 +107,7 @@ extern "C" int mho_host_free(void* ptr) {
 extern "C" int64_t mho_launch_count(const mho_ctx_t* c) { return c ? c->launches : 0; }
 
 extern "C" int mho_invalidate_weights(mho_ctx_t* c) {
-    if (c) { c->wprep_valid = false; c->wdense_valid = false; c->wf16_valid = false; c->wmlp_valid = false; c->wmb_valid = false; }
-    return MHO_OK;
-}
-
-// (Re)build the packed TF32 hi/lo weight images of the CSR-walk kernel when the layer set or the weights changed.
-static int ensure_prepared(mho_ctx* c, const mho_layer_t* layers, int n_layers, const LayerDev* ld, cudaStream_t st) {
-    bool same = c->wprep_valid && (int)c->wkey.size() == n_layers;
-    for (int l = 0; same && l < n_layers; ++l) {
-        mho_wkey k{layers[l].W, layers[l].b, layers[l].K, layers[l].f_in, layers[l].f_out};
-        same = (k == c->wkey[l]);
-    }
-    if (same) return MHO_OK;
-    int rows = 0;
-    for (int l = 0; l < n_layers; ++l) { c->wprep_row_off[l] = rows; rows += wprep_layer_rows(layers[l].K, layers[l].f_out); }
-    const size_t bytes = (size_t)rows * 128;
-    if (bytes > c->wprep_bytes) {
-        if (c->wprep) cudaFree(c->wprep);
-        c->wprep = nullptr; c->wprep_bytes = 0;
-        if (cudaMalloc((void**)&c->wprep, bytes) != cudaSuccess) { mho_set_error("cudaMalloc(%zu) for prepared weights failed", bytes); return MHO_ERR_CUDA; }
-        c->wprep_bytes = bytes;
-    }
-    cudaError_t e = prepare_weights_launch(ld, n_layers, c->wprep_row_off, c->wprep, st);
-    if (e != cudaSuccess) { mho_set_error("prepare_weights launch failed: %s", cudaGetErrorString(e)); return MHO_ERR_CUDA; }
-    c->launches += 1;
-    c->wkey.clear();
-    for (int l = 0; l < n_layers; ++l) c->wkey.push_back(mho_wkey{layers[l].W, layers[l].b, layers[l].K, layers[l].f_in, layers[l].f_out});
-    c->wprep_valid = true;
-    return MHO_OK;
-}
-
-static int ensure_prepared_dense(mho_ctx* c, const mho_layer_t* layers, int n_layers, const LayerDev* ld, cudaStream_t st) {
-    bool same = c->wdense_valid && (int)c->wdkey.size() == n_layers;
-    for (int l = 0; same && l < n_layers; ++l) {
-        mho_wkey k{layers[l].W, layers[l].b, layers[l].K, layers[l].f_in, layers[l].f_out};
-        same = (k == c->wdkey[l]);
-    }
-    if (same) return MHO_OK;
-    c->wd_bytes = cheb_dense_weight_bytes(layers, n_layers, c->wd_off);
-    const size_t bytes = (size_t)c->wd_bytes;
-    if (bytes > c->wdense_bytes) {
-        if (c->wdense) CUDA_TRY(cudaFree(c->wdense));
-        c->wdense = nullptr; c->wdense_bytes = 0;
-        if (cudaMalloc((void**)&c->wdense, bytes) != cudaSuccess) { mho_set_error("cudaMalloc(%zu) for prepared weights failed", bytes); return MHO_ERR_CUDA; }
-        c->wdense_bytes = bytes;
-    }
-    if (cudaMemsetAsync(c->wdense, 0, bytes, st) != cudaSuccess) { mho_set_error("cudaMemsetAsync for prepared weights failed"); return MHO_ERR_CUDA; }
-    cudaError_t e = prepare_dense_weights_launch(ld, n_layers, c->wd_off, c->wdense, st);
-    if (e != cudaSuccess) { mho_set_error("prepare_dense_weights launch failed: %s", cudaGetErrorString(e)); return MHO_ERR_CUDA; }
-    c->launches += 1;
-    c->wdkey.clear();
-    for (int l = 0; l < n_layers; ++l) c->wdkey.push_back(mho_wkey{layers[l].W, layers[l].b, layers[l].K, layers[l].f_in, layers[l].f_out});
-    c->wdense_valid = true;
-    return MHO_OK;
-}
-
-static int ensure_prepared_mlp(mho_ctx* c, const mho_layer_t* layers, int n_layers, const LayerDev* ld, cudaStream_t st) {
-    bool same = c->wmlp_valid && (int)c->wmkey.size() == n_layers;
-    for (int l = 0; same && l < n_layers; ++l) {
-        mho_wkey k{layers[l].W, layers[l].b, layers[l].K, layers[l].f_in, layers[l].f_out};
-        same = (k == c->wmkey[l]);
-    }
-    if (same) return MHO_OK;
-    const size_t bytes = (size_t)cheb_mlp_weight_bytes(n_layers);
-    if (bytes > c->wmlp_bytes) {
-        if (c->wmlp) CUDA_TRY(cudaFree(c->wmlp));
-        c->wmlp = nullptr; c->wmlp_bytes = 0;
-        if (cudaMalloc((void**)&c->wmlp, bytes) != cudaSuccess) { mho_set_error("cudaMalloc(%zu) for prepared weights failed", bytes); return MHO_ERR_CUDA; }
-        c->wmlp_bytes = bytes;
-    }
-    cudaError_t e = prepare_mlp_weights_launch(ld, n_layers, c->wmlp, st);
-    if (e != cudaSuccess) { mho_set_error("prepare_mlp_weights launch failed: %s", cudaGetErrorString(e)); return MHO_ERR_CUDA; }
-    c->launches += 1;
-    c->wmkey.clear();
-    for (int l = 0; l < n_layers; ++l) c->wmkey.push_back(mho_wkey{layers[l].W, layers[l].b, layers[l].K, layers[l].f_in, layers[l].f_out});
-    c->wmlp_valid = true;
-    return MHO_OK;
-}
-
-static int ensure_prepared_f16(mho_ctx* c, const mho_layer_t& L, const LayerDev& ld, cudaStream_t st) {
-    const mho_wkey k{L.W, L.b, L.K, L.f_in, L.f_out};
-    if (c->wf16_valid && k == c->wfkey) return MHO_OK;
-    const size_t bytes = (size_t)cheb_f16_weight_bytes(L.K);
-    if (bytes > c->wf16_bytes) {
-        if (c->wf16) cudaFree(c->wf16);
-        c->wf16 = nullptr; c->wf16_bytes = 0;
-        if (cudaMalloc((void**)&c->wf16, bytes) != cudaSuccess) { mho_set_error("cudaMalloc(%zu) for prepared weights failed", bytes); return MHO_ERR_CUDA; }
-        c->wf16_bytes = bytes;
-    }
-    if (cudaMemsetAsync(c->wf16, 0, bytes, st) != cudaSuccess) { mho_set_error("cudaMemsetAsync for prepared weights failed"); return MHO_ERR_CUDA; }
-    cudaError_t e = prepare_f16_weights_launch(ld, c->wf16, st);
-    if (e != cudaSuccess) { mho_set_error("prepare_f16_weights launch failed: %s", cudaGetErrorString(e)); return MHO_ERR_CUDA; }
-    c->launches += 1;
-    c->wfkey = k;
-    c->wf16_valid = true;
+    if (c) for (auto& im : c->img) im.valid = false;
     return MHO_OK;
 }
 
@@ -266,7 +169,7 @@ extern "C" int mho_fill_tile_info(const int32_t* goff, const int32_t* rowptr, co
 }
 
 // ---------------------------------------------------------------------------------------------
-static int validate_layers(const mho_layer_t* layers, int n_layers, const char* who) {
+int validate_layers(const mho_layer_t* layers, int n_layers, const char* who) {
     if (!layers || n_layers < 1 || n_layers > MHO_MAX_LAYERS) { mho_set_error("%s: n_layers=%d not in [1,%d]", who, n_layers, MHO_MAX_LAYERS); return MHO_ERR_INVALID; }
     for (int l = 0; l < n_layers; ++l) {
         const mho_layer_t& L = layers[l];
@@ -360,10 +263,12 @@ extern "C" int mho_cheb_forward(mho_ctx_t* c, const mho_batch_t* b, const mho_la
     if (b->tile_off && b->tile_info &&
         cheb_f16_eligible(layers, n_layers, b->vals != nullptr, b->adj_bits != nullptr, saved != nullptr && n_layers > 1 /* one layer keeps nothing */, b->tile_graph0 != nullptr && b->graph_off != nullptr,
                           b->max_tile_rows, b->max_tile_nnz, X, Y, b->adj_bits, c->max_smem_optin)) {
-        rc = ensure_prepared_f16(c, layers[0], p.layers[0], (cudaStream_t)stream);
+        auto& img = c->img[MHO_IMG_F16];
+        rc = ensure_image(c, img, layers, 1, (size_t)cheb_f16_weight_bytes(layers[0].K), "prepare_f16_weights",
+                          [&](unsigned char* out) { return prepare_f16_weights_launch(p.layers[0], out, (cudaStream_t)stream); });
         if (rc) return rc;
         dbg_check("f16 prepared");
-        cudaError_t e = cheb_f16_launch(p, c->wf16, b->max_tile_nnz, c->num_sms, c->max_smem_optin, (cudaStream_t)stream);
+        cudaError_t e = cheb_f16_launch(p, img.ptr, b->max_tile_nnz, c->num_sms, c->max_smem_optin, (cudaStream_t)stream);
         dbg_check("f16 launched");
         if (e != cudaSuccess) { mho_set_error("cheb_f16 launch failed: %s", cudaGetErrorString(e)); return MHO_ERR_CUDA; }
         c->launches += 1;
@@ -371,9 +276,11 @@ extern "C" int mho_cheb_forward(mho_ctx_t* c, const mho_batch_t* b, const mho_la
     }
     // stacks whose layers all have K = 1 (the model the reference ships): fused per-row MLP kernel, fp16 parts
     if (b->tile_off && b->tile_info && cheb_mlp_eligible(layers, n_layers, b->max_tile_rows, X, c->max_smem_optin)) {
-        rc = ensure_prepared_mlp(c, layers, n_layers, p.layers, (cudaStream_t)stream);
+        auto& img = c->img[MHO_IMG_MLP];
+        rc = ensure_image(c, img, layers, n_layers, (size_t)cheb_mlp_weight_bytes(n_layers), "prepare_mlp_weights",
+                          [&](unsigned char* out) { return prepare_mlp_weights_launch(p.layers, n_layers, out, (cudaStream_t)stream); });
         if (rc) return rc;
-        cudaError_t e = cheb_mlp_launch(p, c->wmlp, c->num_sms, (cudaStream_t)stream);
+        cudaError_t e = cheb_mlp_launch(p, img.ptr, c->num_sms, (cudaStream_t)stream);
         if (e != cudaSuccess) { mho_set_error("cheb_mlp launch failed: %s", cudaGetErrorString(e)); return MHO_ERR_CUDA; }
         c->launches += 1;
         return MHO_OK;
@@ -381,18 +288,25 @@ extern "C" int mho_cheb_forward(mho_ctx_t* c, const mho_batch_t* b, const mho_la
     // dense-adjacency tcgen05 path (binary adjacency, tiles <= 128 nodes, <= 32 features per layer, stacks)
     if (b->tile_off && b->tile_info && c->sched &&
         cheb_dense_eligible(layers, n_layers, b->vals != nullptr, b->adj_bits != nullptr, b->max_tile_rows, b->max_tile_nnz, c->max_smem_optin)) {
-        rc = ensure_prepared_dense(c, layers, n_layers, p.layers, (cudaStream_t)stream);
+        auto& img = c->img[MHO_IMG_DENSE];
+        int w_off[MHO_MAX_LAYERS];
+        const int w_bytes = cheb_dense_weight_bytes(layers, n_layers, w_off);
+        rc = ensure_image(c, img, layers, n_layers, (size_t)w_bytes, "prepare_dense_weights",
+                          [&](unsigned char* out) { return prepare_dense_weights_launch(p.layers, n_layers, w_off, out, (cudaStream_t)stream); });
         if (rc) return rc;
-        cudaError_t e = cheb_dense_launch(p, c->wdense, c->wd_off, c->wd_bytes, b->max_tile_nnz, c->num_sms, (cudaStream_t)stream);
+        cudaError_t e = cheb_dense_launch(p, img.ptr, w_off, w_bytes, b->max_tile_nnz, c->num_sms, (cudaStream_t)stream);
         dbg_check("dense launched");
         if (e != cudaSuccess) { mho_set_error("cheb_dense launch failed: %s", cudaGetErrorString(e)); return MHO_ERR_CUDA; }
         c->launches += 1;
         return MHO_OK;
     }
-    rc = ensure_prepared(c, layers, n_layers, p.layers, (cudaStream_t)stream);
+    int rows = 0;
+    for (int l = 0; l < n_layers; ++l) { p.wprep_row_off[l] = rows; rows += wprep_layer_rows(layers[l].K, layers[l].f_out); }
+    auto& img = c->img[MHO_IMG_WALK];
+    rc = ensure_image(c, img, layers, n_layers, (size_t)rows * 128, "prepare_weights",
+                      [&](unsigned char* out) { return prepare_weights_launch(p.layers, n_layers, p.wprep_row_off, out, (cudaStream_t)stream); });
     if (rc) return rc;
-    p.wprep = c->wprep;
-    for (int l = 0; l < n_layers; ++l) p.wprep_row_off[l] = c->wprep_row_off[l];
+    p.wprep = img.ptr;
     bool too_large = false;
     cudaError_t e = cheb_forward_launch(p, b->max_tile_rows, b->max_tile_nnz, c->num_sms, c->max_smem_optin,
                                         (cudaStream_t)stream, &too_large);
@@ -454,9 +368,6 @@ static int forward_host_impl(mho_ctx_t* c, int32_t n_graphs, const int32_t* goff
     // chunks: contiguous runs of tiles of roughly equal bytes, ~300 tiles each (measured: copies of a few MB keep both
     // PCIe directions efficient; 2 chunks beat 1, 3 and 4 for the 594-tile benchmark batch), at most 8 chunks
     int n_chunks = (n_tiles + 150) / 300;
-    static int env_chunks = -1;
-    if (env_chunks < 0) { const char* e = getenv("MHO_CHUNKS"); env_chunks = e ? atoi(e) : 0; }  // tuning knob
-    if (env_chunks > 0) n_chunks = env_chunks;
     if (n_chunks > n_tiles) n_chunks = n_tiles;
     if (n_chunks < 1) n_chunks = 1;
     if (n_chunks > 8) n_chunks = 8;

@@ -257,5 +257,34 @@ struct FwdParams {
     int prefetch;     // 1: third tile buffer + second CSR staging set, next tile fetched with cp.async
     int total_nodes;
     int tc5;          // 1: dense part on tcgen05.mma (TMEM accumulators); needs rows_cap <= 128
-    int debug;        // MHO_DEBUG env (perf experiments only): 1 skip sparse step, 2 skip mma, 8 no prefetch
 };
+
+// ---------------------------------------------------------------------------------------------
+// Launch Kernel<<<grid, block, smem, st>>>(args...).  pdl: programmatic dependent launch - the kernel may start
+// while the previous one in the stream drains, so it must execute griddepcontrol.wait before it reads that
+// kernel's results.  The dynamic shared memory limit is sticky per (kernel, device): it is raised only when a
+// launch needs more than the default 48 KB and more than an earlier launch on the same device set.
+// ---------------------------------------------------------------------------------------------
+template <auto Kernel, typename... Args>
+cudaError_t mho_launch(dim3 grid, dim3 block, size_t smem, cudaStream_t st, bool pdl, Args... args) {
+    static int smem_set[64] = {0};
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e != cudaSuccess) return e;
+    if (smem > 48 * 1024 && (int)smem > smem_set[dev & 63]) {
+        e = cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+        smem_set[dev & 63] = (int)smem;
+    }
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = grid;
+    cfg.blockDim = block;
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = st;
+    cfg.attrs = attr;
+    cfg.numAttrs = pdl ? 1 : 0;
+    return cudaLaunchKernelEx(&cfg, Kernel, args...);
+}

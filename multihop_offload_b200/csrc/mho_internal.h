@@ -16,6 +16,17 @@ struct mho_wkey {
     bool operator==(const mho_wkey& o) const { return W == o.W && b == o.b && K == o.K && f_in == o.f_in && f_out == o.f_out; }
 };
 
+// A kernel family's device image of the weights of a layer stack (split / transposed / padded parts, bias).
+// Cached under the stack's weight pointers and shapes; mho_invalidate_weights drops every image, because the
+// optimizer rewrites the weights in place.
+struct mho_wimage {
+    std::vector<mho_wkey> key;
+    bool valid = false;
+    unsigned char* ptr = nullptr;
+    size_t bytes = 0;
+};
+enum { MHO_IMG_WALK, MHO_IMG_DENSE, MHO_IMG_F16, MHO_IMG_MLP, MHO_IMG_MLP_BWD, MHO_N_IMAGES };
+
 #define MHO_MAX_CHUNKS 8
 #define MHO_EV_PER_SLOT (2 * MHO_MAX_CHUNKS + 2)   // per staging slot: upload / kernel events per chunk, start, done
 
@@ -25,34 +36,10 @@ struct mho_ctx {
     cudaEvent_t ev[2 * MHO_EV_PER_SLOT] = {};
     int64_t host_calls = 0;          // host-buffer calls so far: call i uses staging slot i & 1
     bool slot_used[2] = {false, false};
-    // prepared-weight cache (see mho_invalidate_weights)
-    std::vector<mho_wkey> wkey;
-    bool wprep_valid = false;
-    unsigned char* wprep = nullptr;
-    size_t wprep_bytes = 0;
-    int wprep_row_off[MHO_MAX_LAYERS] = {0};
-    // bf16-part weight images of the dense-adjacency tcgen05 path (cheb_forward_dense.cu), cached the same way
-    std::vector<mho_wkey> wdkey;
-    bool wdense_valid = false;
-    unsigned char* wdense = nullptr;
-    size_t wdense_bytes = 0;
-    int wd_off[MHO_MAX_LAYERS] = {0};
-    int wd_bytes = 0;
-    // fp16 two-part weight image of the second-generation dense kernel (cheb_forward_f16.cu), cached the same way
-    mho_wkey wfkey = {nullptr, nullptr, 0, 0, 0};
-    bool wf16_valid = false;
-    unsigned char* wf16 = nullptr;
-    size_t wf16_bytes = 0;
-    // fp16 weight images of the fused K = 1 stack kernel (cheb_mlp_f16.cu)
-    std::vector<mho_wkey> wmkey;
-    bool wmlp_valid = false;
-    unsigned char* wmlp = nullptr;
-    size_t wmlp_bytes = 0;
-    // fp16 W^T images of the K = 1 stack VJP (cheb_mlp_backward_f16.cu)
-    std::vector<mho_wkey> wbkey;
-    bool wmb_valid = false;
-    unsigned char* wmb = nullptr;
-    size_t wmb_bytes = 0;
+    // prepared weights: TF32 hi/lo images of the CSR-walk kernel (cheb_forward.cu), bf16 parts of the dense-adjacency
+    // kernel (cheb_forward_dense.cu), fp16 parts of the one-layer tensor-core kernel (cheb_forward_f16.cu), fp16 images
+    // of the fused K = 1 stack kernel (cheb_mlp_f16.cu) and fp16 W^T images of its VJP (cheb_mlp_backward_f16.cu)
+    mho_wimage img[MHO_N_IMAGES];
     int* sched = nullptr;  // two zero-initialised ints: dynamic tile scheduler state (self re-arming)
     int device = 0;
     int num_sms = 0;
@@ -63,6 +50,31 @@ struct mho_ctx {
 
 void mho_set_error(const char* fmt, ...);
 void* mho_scratch(mho_ctx* c, int slot, size_t bytes);
+int validate_layers(const mho_layer_t* layers, int n_layers, const char* who);
+
+// Make `img` hold the image of `layers` (n_layers entries), `bytes` long: unless it was built from the same stack,
+// (re)allocate it and enqueue prep(img.ptr), which counts as one launch.  `what` names the prep launch in errors.
+template <class Prep>
+int ensure_image(mho_ctx* c, mho_wimage& img, const mho_layer_t* layers, int n_layers, size_t bytes, const char* what, Prep prep) {
+    bool same = img.valid && (int)img.key.size() == n_layers;
+    for (int l = 0; same && l < n_layers; ++l)
+        same = img.key[l] == mho_wkey{layers[l].W, layers[l].b, layers[l].K, layers[l].f_in, layers[l].f_out};
+    if (same) return MHO_OK;
+    img.valid = false;
+    if (bytes > img.bytes) {
+        if (img.ptr) cudaFree(img.ptr);
+        img.ptr = nullptr; img.bytes = 0;
+        if (cudaMalloc((void**)&img.ptr, bytes) != cudaSuccess) { mho_set_error("cudaMalloc(%zu) for prepared weights failed", bytes); return MHO_ERR_CUDA; }
+        img.bytes = bytes;
+    }
+    const cudaError_t e = prep(img.ptr);
+    if (e != cudaSuccess) { mho_set_error("%s launch failed: %s", what, cudaGetErrorString(e)); return MHO_ERR_CUDA; }
+    c->launches += 1;
+    img.key.clear();
+    for (int l = 0; l < n_layers; ++l) img.key.push_back(mho_wkey{layers[l].W, layers[l].b, layers[l].K, layers[l].f_in, layers[l].f_out});
+    img.valid = true;
+    return MHO_OK;
+}
 
 struct LayerDev;
 struct FwdParams;

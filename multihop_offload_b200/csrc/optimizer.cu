@@ -132,6 +132,6 @@ extern "C" int mho_adam_replay(mho_ctx_t* c, const mho_layer_t* layers, int32_t 
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) { mho_set_error("adam_replay launch failed: %s", cudaGetErrorString(e)); return MHO_ERR_CUDA; }
     c->launches += 1;
-    c->wprep_valid = false; c->wdense_valid = false; c->wf16_valid = false; c->wmlp_valid = false; c->wmb_valid = false;  // params_f32 changed in place: the packed weight images are stale
+    mho_invalidate_weights(c);  // params_f32 changed in place: the packed weight images are stale
     return MHO_OK;
 }

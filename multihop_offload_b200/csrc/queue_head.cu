@@ -160,13 +160,10 @@ extern "C" int mho_queue_head_forward(mho_ctx_t* c, const mho_head_t* hd, const 
     if (!lam || !link_delay || !node_delay) { mho_set_error("mho_queue_head_forward: NULL buffer"); return MHO_ERR_INVALID; }
     if (cudaSetDevice(c->device) != cudaSuccess) { mho_set_error("cudaSetDevice failed"); return MHO_ERR_CUDA; }
     const size_t smem = (size_t)3 * hd->max_links * sizeof(double) + 16;
-    if (smem > 48 * 1024) {
-        if (smem > (size_t)c->max_smem_optin) { mho_set_error("mho_queue_head_forward: %d links per graph exceed shared memory", hd->max_links); return MHO_ERR_TOO_LARGE; }
-        cudaFuncSetAttribute(queue_head_forward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    }
+    if (smem > (size_t)c->max_smem_optin) { mho_set_error("mho_queue_head_forward: %d links per graph exceed shared memory", hd->max_links); return MHO_ERR_TOO_LARGE; }
     int grid = hd->n_graphs < 8 * c->num_sms ? hd->n_graphs : 8 * c->num_sms;
-    queue_head_forward_kernel<<<grid, QH_THREADS, smem, (cudaStream_t)stream>>>(h, lam, link_delay, node_delay, saved_mu, hd->total_links);
-    cudaError_t e = cudaGetLastError();
+    cudaError_t e = mho_launch<queue_head_forward_kernel>(dim3((unsigned)grid), dim3(QH_THREADS), smem, (cudaStream_t)stream, false, h, lam, link_delay,
+                                                           node_delay, saved_mu, hd->total_links);
     if (e != cudaSuccess) { mho_set_error("queue_head_forward launch failed: %s", cudaGetErrorString(e)); return MHO_ERR_CUDA; }
     c->launches += 1;
     return MHO_OK;
@@ -182,13 +179,10 @@ extern "C" int mho_queue_head_backward(mho_ctx_t* c, const mho_head_t* hd, const
     if (!lam || !saved_mu || !g_link || !g_node || !g_lam) { mho_set_error("mho_queue_head_backward: NULL buffer"); return MHO_ERR_INVALID; }
     if (cudaSetDevice(c->device) != cudaSuccess) { mho_set_error("cudaSetDevice failed"); return MHO_ERR_CUDA; }
     const size_t smem = (size_t)5 * hd->max_links * sizeof(double) + 16;
-    if (smem > 48 * 1024) {
-        if (smem > (size_t)c->max_smem_optin) { mho_set_error("mho_queue_head_backward: %d links per graph exceed shared memory", hd->max_links); return MHO_ERR_TOO_LARGE; }
-        cudaFuncSetAttribute(queue_head_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    }
+    if (smem > (size_t)c->max_smem_optin) { mho_set_error("mho_queue_head_backward: %d links per graph exceed shared memory", hd->max_links); return MHO_ERR_TOO_LARGE; }
     int grid = hd->n_graphs < 8 * c->num_sms ? hd->n_graphs : 8 * c->num_sms;
-    queue_head_backward_kernel<<<grid, QH_THREADS, smem, (cudaStream_t)stream>>>(h, lam, saved_mu, g_link, g_node, g_lam, hd->total_links);
-    cudaError_t e = cudaGetLastError();
+    cudaError_t e = mho_launch<queue_head_backward_kernel>(dim3((unsigned)grid), dim3(QH_THREADS), smem, (cudaStream_t)stream, false, h, lam, saved_mu,
+                                                            g_link, g_node, g_lam, hd->total_links);
     if (e != cudaSuccess) { mho_set_error("queue_head_backward launch failed: %s", cudaGetErrorString(e)); return MHO_ERR_CUDA; }
     c->launches += 1;
     return MHO_OK;

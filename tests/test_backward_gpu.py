@@ -108,6 +108,27 @@ def test_backward_golden_rollout_cases(torch_cuda, golden_dir):
                 assert rel_err(dX, z["dX_K3"]) < GTOL
 
 
+def test_backward_rejects_invalid_layer_stacks(torch_cuda):
+    """mho_cheb_backward checks the layer stack as mho_cheb_forward does: widths that do not chain and an unknown activation
+    are MHO_ERR_INVALID, and nothing is launched.  The batch has no graphs and the gradient buffers are NULL, so an accepted
+    stack would not launch or write anything either."""
+    import ctypes as C
+    from multihop_offload_b200 import _lib
+    ctx = _lib.Context.get(0)
+    buf = torch_cuda.zeros(4096, dtype=torch_cuda.float32, device="cuda:0")
+    offs = torch_cuda.zeros(1, dtype=torch_cuda.int32, device="cuda:0")
+    b = _lib.mho_batch_t()
+    b.graph_off = offs.data_ptr(); b.rowptr = offs.data_ptr(); b.max_tile_rows = 1
+    p = buf.data_ptr()
+    before = ctx.launch_count()
+    for layers in ([(3, 32, 16, O.ACT_LEAKY), (2, 8, 1, O.ACT_RELU)],   # f_in 8 != previous f_out 16
+                   [(3, 32, 32, 3)]):                                  # act 3 does not exist
+        arr = (_lib.mho_layer_t * len(layers))(*[_lib.mho_layer_t(K, fi, fo, act, 0.2, p, p) for K, fi, fo, act in layers])
+        rc = ctx.lib.mho_cheb_backward(ctx.handle, C.byref(b), arr, len(layers), p, p, p, p, None, None, None, None)
+        assert rc == -1, (layers, rc)   # MHO_ERR_INVALID
+    assert ctx.launch_count() == before
+
+
 def test_adam_replay_matches_keras_semantics(torch_cuda):
     from multihop_offload_b200 import ChebNet, reference_stack
     from multihop_offload_b200.optim import KerasAdamReplay

@@ -1,5 +1,5 @@
-"""Worst per-block relative error of the VJP (vs the fp64 numpy oracle) per order K, for the kernel the library picks
-(MHO_DEBUG=512: the CUDA-core kernel).  Debug aid for tests/test_backward_f16_gpu.py; run from the repo root."""
+"""Worst per-block relative error of the VJP (vs the fp64 numpy oracle) per order K, for the kernel the library picks.
+Debug aid for tests/test_backward_f16_gpu.py; run from the repo root."""
 import sys, os
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests")); sys.path.insert(0, os.path.join(ROOT, "oracle"))

@@ -1,4 +1,4 @@
-"""e2e probe: time mho_cheb_forward_host with different chunk counts (MHO_CHUNKS env is read once per process)."""
+"""e2e probe: time mho_cheb_forward_host on the benchmark batch from page-locked buffers."""
 import os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch, bench
@@ -15,4 +15,4 @@ def step():
 for _ in range(5): step()
 t = time.perf_counter()
 for _ in range(30): step()
-print("chunks", os.environ.get("MHO_CHUNKS"), "us/step %.1f" % ((time.perf_counter() - t) / 30 * 1e6))
+print("us/step %.1f" % ((time.perf_counter() - t) / 30 * 1e6))

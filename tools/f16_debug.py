@@ -1,6 +1,5 @@
 """Debug probe for the fp16-parts forward kernel (cheb_forward_f16.cu): one 32->32 layer, K given on the command line,
-small and full-size batches, with bit rows and with CSR input; prints the per-graph error against the fp64 oracle and the
-same for the first-generation dense kernel (MHO_DEBUG=64 in a second process)."""
+small and full-size batches, with bit rows and with CSR input; prints the per-graph error against the fp64 oracle."""
 import os, sys, time
 import numpy as np, torch
 sys.path.insert(0, os.path.join(os.path.dirname(__file__), "..", "tests"))

@@ -1,5 +1,5 @@
 """Long CTA pipelines (many tiles / graphs per CTA): writes the forward output and the VJP gradients of a big batch to an .npz.
-usage: stress_long.py out.npz [graphs=8192] [K=5]   (run twice with different MHO_WS / MHO_DEBUG and compare)"""
+usage: stress_long.py out.npz [graphs=8192] [K=5]   (run against two builds, MHO_LIB=..., and compare)"""
 import sys, os
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch, bench
