@@ -213,6 +213,73 @@ int mho_queue_head_backward(mho_ctx_t* ctx, const mho_head_t* head, const float*
 int mho_apsp(mho_ctx_t* ctx, int32_t n_graphs, const int32_t* node_off, const int32_t* rowptr, const int32_t* colidx,
              const double* weight, const int64_t* out_off, double* dist, mho_stream_t stream);
 
+/* ---- environment step: replaces AdhocCloud.offloading(sp, hop) with explore = 0, prob = False (src/offloading_v3.py:388-453)
+ * or AdhocCloud.local_compute(dproc) (:363-386), followed by AdhocCloud.run() (:455-550) and the drivers'
+ * delay_emp = nansum(delay_links, 0) + nansum(delay_nodes, 0) (AdHoc_test.py:140-153), for a batch of ITEMS: one item is
+ * one (network, job set, method).  fp64 throughout, bit-identical to the reference (no contracted multiply-adds; the
+ * sums follow numpy's summation order).  One CTA per item.
+ *
+ * Networks are concatenated like mho_head_t; every id stored in the arrays is LOCAL to its network.  Per network g:
+ * nodes [node_off[g], node_off[g+1]), links [link_off[g], link_off[g+1]) in env.link_list order, servers
+ * [server_off[g], server_off[g+1]) in env.servers order.  adj_rowptr [total_nodes+1] (global offsets) / adj_col /
+ * adj_link: env.adj_c row by row in its stored CSR order without explicit zeros (what np.nonzero(adj_c[v]) returns),
+ * adj_link = the env.link_list index of (v, u), else of (u, v), else -1.  cf_rowptr [total_links+1] (global offsets) /
+ * cf_col: the binary conflict graph env.adj_i, neighbours in ASCENDING order.  hop: one row-major n x n block per network
+ * at element offset hop_off[g] (the hop-count shortest paths, instance-invariant). */
+enum { MHO_ENV_MAX_NODES = 512, MHO_ENV_MAX_LINKS = 1024, MHO_ENV_MAX_JOBS = 512 };
+enum { MHO_ENV_GREEDY = 0, MHO_ENV_LOCAL = 1 };
+/* per-item status */
+enum {
+    MHO_ENV_OK = 0,
+    MHO_ENV_ROUTE_LOOP = 1,   /* a route walk did not reach its server within n hops (the reference never returns) */
+    MHO_ENV_NO_LINK = 2,      /* a route walk met a node without neighbours or an adjacency entry without a link id
+                                 (the reference raises ValueError) */
+    MHO_ENV_BAD_ITEM = 3      /* network index, mode, job range, source node or a size beyond the MHO_ENV_MAX_* limits */
+};
+typedef struct {
+    int32_t n_nets;
+    int32_t max_nodes, max_links;            /* host-known maxima over the networks (limits and shared-memory sizing) */
+    const int32_t* node_off; const int32_t* link_off; const int32_t* server_off;   /* [n_nets+1] */
+    const int32_t* servers;                  /* [total_servers] */
+    const int32_t* adj_rowptr; const int32_t* adj_col; const int32_t* adj_link;
+    const double* link_rates; const double* cf_degs;                             /* [total_links] */
+    const double* proc_bws;                  /* [total_nodes] */
+    const int32_t* cf_rowptr; const int32_t* cf_col;
+    const double* hop; const int64_t* hop_off;
+    const double* T;                         /* [n_nets] env.T */
+} mho_env_t;
+/* Item i: network net[i], mode[i], jobs [job_off[i], job_off[i+1]) in env.jobs order (source node, arrival rate, ul_data,
+ * dl_data), and the n x n fp64 shortest-path block at element offset sp_off[i] of sp, row-major as mho_apsp writes it
+ * and with the server unit delays on the diagonal (the matrix the reference passes to offloading()).  Items may share
+ * a block.  MHO_ENV_LOCAL reads only its diagonal (the dproc of local_compute). */
+typedef struct {
+    int32_t n_items;
+    int32_t max_jobs;                        /* host-known maximum job count of one item */
+    const int32_t* net; const int32_t* mode; const int32_t* job_off;   /* [n_items], [n_items], [n_items+1] */
+    const double* sp; const int64_t* sp_off;
+    const int32_t* src; const double* rate; const double* ul; const double* dl;   /* [total_jobs] */
+} mho_env_items_t;
+/* Per job (global job index): dst (flow.dst), nhop, delay_est (the delay offloading() / local_compute() returns),
+ * delay_emp.  Optional (NULL = not written), each at a per-item ELEMENT offset:
+ *   routes [J][route_stride] int32 at routes_off[i]: flow.route, padded with -1 (route_stride >= n + 1);
+ *   delay_links [L][J] at links_off[i], delay_nodes [n][J] at nodes_off[i], unit [n][n] at unit_off[i]: run()'s three
+ *   matrices, row-major, NaN where run() leaves NaN.
+ * status [n_items] (MHO_ENV_*).  An item whose status is ROUTE_LOOP or NO_LINK gets dst = nhop = -1 and NaN delays for
+ * all its jobs and NaN/-1 in its optional outputs; a BAD_ITEM writes its status only.  Other items are unaffected. */
+typedef struct {
+    int32_t* dst; int32_t* nhop; double* delay_est; double* delay_emp;
+    int32_t* routes; const int64_t* routes_off; int32_t route_stride;
+    double* delay_links; const int64_t* links_off;
+    double* delay_nodes; const int64_t* nodes_off;
+    double* unit; const int64_t* unit_off;
+    int32_t* status;
+} mho_env_out_t;
+/* MHO_ERR_INVALID on a NULL required pointer, an optional output without its offsets or a negative count;
+ * MHO_ERR_TOO_LARGE when max_nodes / max_links / max_jobs exceed the MHO_ENV_MAX_* limits.  All pointers inside the
+ * three structs are DEVICE memory; the structs themselves are host memory. */
+int mho_env_step(mho_ctx_t* ctx, const mho_env_t* nets, const mho_env_items_t* items, const mho_env_out_t* out,
+                 mho_stream_t stream);
+
 /* ---- host-buffer convenience (the reference-facing call: numpy in, numpy out, as
  * ACOAgent.predict takes them).  All pointers are HOST memory (pinned for full speed); the
  * call uploads the batch + X, runs mho_cheb_forward, downloads Y and synchronises `stream`.

@@ -9,6 +9,9 @@ _LIB = None
 
 ACT_NONE, ACT_RELU, ACT_LEAKY = 0, 1, 2
 MAX_F, MAX_K, MAX_LAYERS, MAX_TILE_ROWS = 32, 16, 16, 512
+ENV_MAX_NODES, ENV_MAX_LINKS, ENV_MAX_JOBS = 512, 1024, 512
+ENV_GREEDY, ENV_LOCAL = 0, 1
+ENV_OK, ENV_ROUTE_LOOP, ENV_NO_LINK, ENV_BAD_ITEM = 0, 1, 2, 3
 
 
 class MhoError(RuntimeError):
@@ -35,6 +38,28 @@ class mho_head_t(C.Structure):
                 ("total_adj_nnz", C.c_int64), ("ext_off", C.c_void_p), ("link_off", C.c_void_p), ("comp_off", C.c_void_p),
                 ("maps_ol_el", C.c_void_p), ("maps_on_el", C.c_void_p), ("link_rates", C.c_void_p), ("cf_degs", C.c_void_p),
                 ("node_mu", C.c_void_p), ("adj_rowptr", C.c_void_p), ("adj_colidx", C.c_void_p), ("T", C.c_double)]
+
+
+class mho_env_t(C.Structure):
+    _fields_ = [("n_nets", C.c_int32), ("max_nodes", C.c_int32), ("max_links", C.c_int32),
+                ("node_off", C.c_void_p), ("link_off", C.c_void_p), ("server_off", C.c_void_p), ("servers", C.c_void_p),
+                ("adj_rowptr", C.c_void_p), ("adj_col", C.c_void_p), ("adj_link", C.c_void_p),
+                ("link_rates", C.c_void_p), ("cf_degs", C.c_void_p), ("proc_bws", C.c_void_p),
+                ("cf_rowptr", C.c_void_p), ("cf_col", C.c_void_p), ("hop", C.c_void_p), ("hop_off", C.c_void_p),
+                ("T", C.c_void_p)]
+
+
+class mho_env_items_t(C.Structure):
+    _fields_ = [("n_items", C.c_int32), ("max_jobs", C.c_int32), ("net", C.c_void_p), ("mode", C.c_void_p),
+                ("job_off", C.c_void_p), ("sp", C.c_void_p), ("sp_off", C.c_void_p), ("src", C.c_void_p),
+                ("rate", C.c_void_p), ("ul", C.c_void_p), ("dl", C.c_void_p)]
+
+
+class mho_env_out_t(C.Structure):
+    _fields_ = [("dst", C.c_void_p), ("nhop", C.c_void_p), ("delay_est", C.c_void_p), ("delay_emp", C.c_void_p),
+                ("routes", C.c_void_p), ("routes_off", C.c_void_p), ("route_stride", C.c_int32),
+                ("delay_links", C.c_void_p), ("links_off", C.c_void_p), ("delay_nodes", C.c_void_p),
+                ("nodes_off", C.c_void_p), ("unit", C.c_void_p), ("unit_off", C.c_void_p), ("status", C.c_void_p)]
 
 
 class mho_adam_t(C.Structure):
@@ -75,6 +100,8 @@ PROTOTYPES = [
     ("mho_host_wait", C.c_int, [C.c_void_p, C.c_int32]),
     ("mho_apsp", C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                            C.c_void_p]),
+    ("mho_env_step", C.c_int, [C.c_void_p, C.POINTER(mho_env_t), C.POINTER(mho_env_items_t), C.POINTER(mho_env_out_t),
+                               C.c_void_p]),
     ("mho_host_alloc", C.c_int, [C.POINTER(C.c_void_p), C.c_size_t]),
     ("mho_host_free", C.c_int, [C.c_void_p]),
     ("mho_cheb_forward_host", C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,

@@ -8,7 +8,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libmho.so")
-SOURCES = ["mho_api.cu", "cheb_forward.cu", "cheb_forward_dense.cu", "cheb_forward_f16.cu", "cheb_mlp_f16.cu", "cheb_backward.cu", "cheb_backward_f16.cu", "cheb_mlp_backward_f16.cu", "optimizer.cu", "queue_head.cu", "apsp.cu"]
+SOURCES = ["mho_api.cu", "cheb_forward.cu", "cheb_forward_dense.cu", "cheb_forward_f16.cu", "cheb_mlp_f16.cu", "cheb_backward.cu", "cheb_backward_f16.cu", "cheb_mlp_backward_f16.cu", "optimizer.cu", "queue_head.cu", "apsp.cu", "env_step.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xptxas=-v", "-Xcompiler", "-fPIC", "-shared"]
 

@@ -92,6 +92,40 @@ extern "C" int mho_apsp(mho_ctx_t* c, int32_t n_graphs, const int32_t* node_off,
     return MHO_OK;
 }
 
+extern "C" int mho_env_step(mho_ctx_t* c, const mho_env_t* nets, const mho_env_items_t* items, const mho_env_out_t* out,
+                            mho_stream_t stream) {
+    if (!c || !nets || !items || !out) { mho_set_error("mho_env_step: NULL argument"); return MHO_ERR_INVALID; }
+    const mho_env_t& E = *nets;
+    const mho_env_items_t& I = *items;
+    const mho_env_out_t& O = *out;
+    if (E.n_nets < 0 || I.n_items < 0 || E.max_nodes < 0 || E.max_links < 0 || I.max_jobs < 0) {
+        mho_set_error("mho_env_step: negative count"); return MHO_ERR_INVALID;
+    }
+    if (I.n_items == 0) return MHO_OK;
+    if (E.n_nets == 0 || !E.node_off || !E.link_off || !E.server_off || !E.adj_rowptr || !E.link_rates || !E.cf_degs ||
+        !E.proc_bws || !E.cf_rowptr || !E.hop || !E.hop_off || !E.T || !I.net || !I.mode || !I.job_off || !I.sp || !I.sp_off ||
+        !O.dst || !O.nhop || !O.delay_est || !O.delay_emp || !O.status) {
+        mho_set_error("mho_env_step: a required pointer is NULL"); return MHO_ERR_INVALID;
+    }
+    if ((O.routes && (!O.routes_off || O.route_stride < E.max_nodes + 1)) || (O.delay_links && !O.links_off) ||
+        (O.delay_nodes && !O.nodes_off) || (O.unit && !O.unit_off)) {
+        mho_set_error("mho_env_step: an optional output lacks its offsets (or route_stride < max_nodes + 1)"); return MHO_ERR_INVALID;
+    }
+    if (E.max_nodes > MHO_ENV_MAX_NODES || E.max_links > MHO_ENV_MAX_LINKS || I.max_jobs > MHO_ENV_MAX_JOBS) {
+        mho_set_error("mho_env_step: %d nodes / %d links / %d jobs exceed the limits %d / %d / %d", E.max_nodes, E.max_links,
+                      I.max_jobs, (int)MHO_ENV_MAX_NODES, (int)MHO_ENV_MAX_LINKS, (int)MHO_ENV_MAX_JOBS);
+        return MHO_ERR_TOO_LARGE;
+    }
+    CUDA_TRY(cudaSetDevice(c->device));
+    if (env_step_smem(E.max_nodes, E.max_links, I.max_jobs) > (size_t)c->max_smem_optin) {
+        mho_set_error("mho_env_step: shared memory need exceeds the device's limit"); return MHO_ERR_TOO_LARGE;
+    }
+    cudaError_t e = env_step_launch(E, I, O, (cudaStream_t)stream);
+    if (e != cudaSuccess) { mho_set_error("env_step launch failed: %s", cudaGetErrorString(e)); return MHO_ERR_CUDA; }
+    c->launches += 1;
+    return MHO_OK;
+}
+
 extern "C" int mho_host_alloc(void** ptr, size_t bytes) {
     if (!ptr) { mho_set_error("mho_host_alloc: ptr is NULL"); return MHO_ERR_INVALID; }
     *ptr = nullptr;

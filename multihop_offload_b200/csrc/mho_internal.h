@@ -109,5 +109,7 @@ cudaError_t cheb_mlp_backward_launch(const mho_batch_t* b, const LayerDev* layer
                                      const float* dY, float* grads, long long n_params, const unsigned char* wT, int num_sms, cudaStream_t st);
 cudaError_t apsp_launch(int n_graphs, const int32_t* node_off, const int32_t* rowptr, const int32_t* colidx, const double* weight,
                         const int64_t* out_off, double* dist, int max_smem_optin, cudaStream_t st);
+size_t env_step_smem(int max_nodes, int max_links, int max_jobs);
+cudaError_t env_step_launch(const mho_env_t& nets, const mho_env_items_t& items, const mho_env_out_t& out, cudaStream_t st);
 cudaError_t cheb_forward_launch(FwdParams& p, int max_tile_rows, int max_tile_nnz, int num_sms, int max_smem_optin,
                                 cudaStream_t st, bool* too_large);
